@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- POIs/sec of the FFT-CC -> IC-GN hot path (BASELINE.json metric) on N B200s.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--config B|C|D|A|E|F] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--config B|C|D|A|E|F] [--impl ours|reference] [--dump-outputs DIR]
   N>1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step = one pass of the hot path (FFT-CC initial guess + IC-GN to convergence, prepare() included)
@@ -89,6 +89,22 @@ def make_workload(cfg_name, rank, world, device=None):
     xyz = synth.grid_3d(x0 + rank, y0, z0, nx, ny, nz, sx, sy, sz)
     cfg["n_poi"] = xyz.shape[0]
     return cfg, ref, tar, xyz
+
+
+DUMP_LIMIT_BYTES = 64 * 1000 * 1000
+
+
+def dump_outputs(out_dir, pois, rank=0, world=1):
+    """--dump-outputs: the POI records the timed path returned in its last step, as out_dir/pois.npy (one rank) or
+    pois_rank<k>.npy, float32 [n, 25] (POI2D) / [n, 31] (POI3D).  Every record carries its own coordinates, so two runs can be
+    matched row for row.  Above this rank's share of DUMP_LIMIT_BYTES a fixed, seeded sample of rows is written, in queue order."""
+    os.makedirs(out_dir, exist_ok=True)
+    pois = np.ascontiguousarray(pois, dtype=np.float32)
+    budget = DUMP_LIMIT_BYTES // world - 4096  # room for the .npy header
+    if pois.nbytes > budget:
+        keep = budget // (pois.shape[1] * 4)
+        pois = pois[np.sort(np.random.default_rng(0).choice(len(pois), keep, replace=False))]
+    np.save(os.path.join(out_dir, "pois.npy" if world == 1 else "pois_rank%d.npy" % rank), pois)
 
 
 def workload_name(cfg_name, cfg):
@@ -196,6 +212,8 @@ def run_reference(args):
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, c["queue"])
     print(json.dumps(line))
     return 0
 
@@ -666,7 +684,7 @@ def run_ours(args):
     e2e_shim, capi_multi, cold = None, None, None
     torch.cuda.synchronize(dev)
     if rank == 0 and not args.no_extras:
-        sub_steps = max(3, min(args.steps, 5))
+        sub_steps = min(args.steps, 5)
         if world == 1:
             e2e_shim = shim_e2e(cfg, ref, tar, sub_steps, 2, {"OPENCORR_B200_DEVICE": str(local_rank)})
             cold = cold_start_record()
@@ -689,6 +707,8 @@ def run_ours(args):
     if idle_group is not None:
         dist.barrier(group=idle_group)
 
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res, rank, world)
     if rank == 0:
         line = {
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
@@ -728,7 +748,11 @@ def main():
     ap.add_argument("--cpu-sample", type=int, default=0, help="POIs per step for --impl reference (0 = default)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the rank-0 extras (e2e_shim, capi_multi, cold_start)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the POI records of the last timed step to DIR/pois.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

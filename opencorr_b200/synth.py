@@ -30,11 +30,20 @@ def _render_torch(shape, centres, amps, rho, device):
     lim = torch.tensor(shape, device=device)
     strides = torch.tensor([int(np.prod(shape[i + 1:])) for i in range(nd)], dtype=torch.int64, device=device)
     inv = 1.0 / (rho * rho)
-    for o in offs:
-        p = base + o
-        ok = ((p >= 0) & (p < lim)).all(1)
-        d2 = ((p[ok].to(torch.float64) - c[ok]) ** 2).sum(1)
-        img.index_add_(0, (p[ok] * strides).sum(1), a[ok] * torch.exp(-d2 * inv))
+    # centres that share a pixel cell add to the same pixel in one index_add_; on CUDA its default atomics add them in a
+    # different order from run to run, and the last bit can round a pixel the other way: deterministic mode fixes the order,
+    # so the same arguments render the same images every time
+    was_deterministic = torch.are_deterministic_algorithms_enabled()
+    was_warn_only = torch.is_deterministic_algorithms_warn_only_enabled()
+    torch.use_deterministic_algorithms(True)
+    try:
+        for o in offs:
+            p = base + o
+            ok = ((p >= 0) & (p < lim)).all(1)
+            d2 = ((p[ok].to(torch.float64) - c[ok]) ** 2).sum(1)
+            img.index_add_(0, (p[ok] * strides).sum(1), a[ok] * torch.exp(-d2 * inv))
+    finally:
+        torch.use_deterministic_algorithms(was_deterministic, warn_only=was_warn_only)
     return img.reshape(shape).cpu().numpy()
 
 

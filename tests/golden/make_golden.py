@@ -1,6 +1,6 @@
 """Regenerates the committed fixtures under tests/golden/ from the reference checkout.
 
-Run in the build container (the GPU box has no /root/reference):  python tests/golden/make_golden.py
+Run where the OpenCorr checkout is (OPENCORR_REF, default /root/reference, as in oracle/Makefile):  python tests/golden/make_golden.py
 Only DATA is copied (images, sub-sampled result tables the reference ships as its regression
 fixtures, examples/2d_dic and examples/dvc); no reference source code.
 
@@ -8,6 +8,8 @@ Outputs
   oht_cfrp_0.bmp, oht_cfrp_4.bmp    the 2D example pair (280x900, 8-bit), verbatim
   oht_cfrp_4_fftcc_icgn1_r16.npz    every 23rd row of the shipped result table + deformation table, plus the three rows whose
                                     FFT-CC guess is an exact tie between two correlation bins (fftcc_tie_rows / fftcc_tie_table)
+  oht_cfrp_4_fftcc_icgn1_r16_full.npz  all 30 000 rows of that table, the columns the oracle is checked on: x, y, u0, v0, iteration
+                                    (int16 / int8) and u, v, ZNCC (float64, as printed)
   oht_cfrp_4_fftcc_iclm1_r16.npz    the same rows of the shipped ICLM2D1 table
   oht_cfrp_4_sift_icgn2_gpu_r16.npz every 23rd row of examples/2d_dic/oht_cfrp_4_sift_icgn2(gpu)_r16.csv (the reference's GPU ICGN2D2,
                                     SIFT-seeded): x,y,u,v,u0,v0,ZNCC,iteration,convergence.  u0, v0 are the seeds; the affine part
@@ -45,7 +47,7 @@ import shutil
 
 import numpy as np
 
-REF = "/root/reference/examples"
+REF = os.path.join(os.environ.get("OPENCORR_REF", "/root/reference"), "examples")
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -164,6 +166,12 @@ def make_epipolar_fixture():
                         fundamental=fm, columns=np.array("x,y,r1r2 ZNCC,r2_x,r2_y".split(",")), table=blk[:, :5])
 
 
+def make_full_2d_table():
+    tab = np.genfromtxt(os.path.join(REF, "2d_dic", "oht_cfrp_4_fftcc_icgn1_r16.csv"), delimiter=",", skip_header=1)
+    np.savez_compressed(os.path.join(OUT, "oht_cfrp_4_fftcc_icgn1_r16_full.npz"), xy=tab[:, 0:2].astype(np.int16),
+                        u0v0=tab[:, 4:6].astype(np.int16), iteration=tab[:, 7].astype(np.int8), uv=tab[:, 2:4], zncc=tab[:, 6])
+
+
 def main():
     for name in ("oht_cfrp_0.bmp", "oht_cfrp_4.bmp"):
         shutil.copyfile(os.path.join(REF, "2d_dic", name), os.path.join(OUT, name))
@@ -178,6 +186,7 @@ def main():
                         columns=np.array("x,y,u,v,u0,v0,ZNCC,iteration,convergence".split(",")),
                         table=tab[sel, :9], deformation_columns=np.array("x,y,u,ux,uy,v,vx,vy".split(",")),
                         deformation=dtab[sel, :8], rows=sel, fftcc_tie_rows=ties, fftcc_tie_table=tab[ties, :9])
+    make_full_2d_table()
 
     # ICLM2D1 table shipped by the reference (examples/2d_dic/oht_cfrp_4_fftcc_iclm1_r16.csv, same POIs)
     itab = np.genfromtxt(os.path.join(REF, "2d_dic", "oht_cfrp_4_fftcc_iclm1_r16.csv"), delimiter=",", skip_header=1)

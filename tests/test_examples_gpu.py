@@ -1,6 +1,7 @@
-"""Acceptance: the reference's own example program, compiled UNCHANGED against the C++ shim
-(examples/Makefile -> examples/bin/test_2d_dic_fftcc_icgn1, built where the reference checkout is
-mounted), runs on the GPU and reproduces the reference's shipped result table."""
+"""Acceptance: the reference's own example programs, compiled UNCHANGED against the C++ shim
+(build() -> oracle/Makefile ref-examples -> oracle/_ref/bin/test_2d_dic_fftcc_icgn1, ..., from the OpenCorr
+checkout), run on the GPU and reproduce the reference's shipped result tables;
+this repo's own shim programs (examples/bin/) run on the committed example pair."""
 import os
 import shutil
 import subprocess
@@ -13,6 +14,8 @@ import util
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BIN = os.path.join(ROOT, "examples", "bin")
+REF_BIN = os.path.join(ROOT, "oracle", "_ref", "bin")
+REF_MISSING = "reference example program not in oracle/_ref/bin/: build() found no OpenCorr checkout (oracle/Makefile, OPENCORR_REF)"
 
 
 def _read_table(path):
@@ -22,13 +25,13 @@ def _read_table(path):
     return header, np.array(rows)
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(BIN, "test_2d_dic_fftcc_icgn1")), reason="example binary not built")
+@pytest.mark.skipif(not os.path.exists(os.path.join(REF_BIN, "test_2d_dic_fftcc_icgn1")), reason=REF_MISSING)
 def test_reference_2d_example_runs_unchanged(tmp_path):
     data = tmp_path / "d:" / "dic_tests" / "2d_dic"  # the example hard-codes d:/dic_tests/2d_dic/...
     data.mkdir(parents=True)
     for name in ("oht_cfrp_0.bmp", "oht_cfrp_4.bmp"):
         shutil.copyfile(os.path.join(util.GOLDEN, name), data / name)
-    out = subprocess.run([os.path.join(BIN, "test_2d_dic_fftcc_icgn1")], cwd=tmp_path, stdin=subprocess.DEVNULL,
+    out = subprocess.run([os.path.join(REF_BIN, "test_2d_dic_fftcc_icgn1")], cwd=tmp_path, stdin=subprocess.DEVNULL,
                          capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stdout + out.stderr
     assert "30000 POIs" in out.stdout
@@ -64,14 +67,14 @@ def test_shim_demo(tmp_path):
     assert tab.shape[0] > 1000 and (tab[:, 6] > 0.9).mean() > 0.9
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(BIN, "test_2d_dic_fftcc_iclm1")), reason="example binary not built")
+@pytest.mark.skipif(not os.path.exists(os.path.join(REF_BIN, "test_2d_dic_fftcc_iclm1")), reason=REF_MISSING)
 def test_reference_2d_iclm_example_runs_unchanged(tmp_path):
     """examples/test_2d_dic_fftcc_iclm1.cpp of the reference, compiled unchanged against the shim."""
     data = tmp_path / "d:" / "dic_tests" / "2d_dic"
     data.mkdir(parents=True)
     for name in ("oht_cfrp_0.bmp", "oht_cfrp_4.bmp"):
         shutil.copyfile(os.path.join(util.GOLDEN, name), data / name)
-    out = subprocess.run([os.path.join(BIN, "test_2d_dic_fftcc_iclm1")], cwd=tmp_path, stdin=subprocess.DEVNULL,
+    out = subprocess.run([os.path.join(REF_BIN, "test_2d_dic_fftcc_iclm1")], cwd=tmp_path, stdin=subprocess.DEVNULL,
                          capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stdout + out.stderr
     _, tab = _read_table(data / "oht_cfrp_4_fftcc_iclm1_r16.csv")
@@ -85,14 +88,14 @@ def test_reference_2d_iclm_example_runs_unchanged(tmp_path):
     assert np.percentile(d, 98) < 1e-4 and d.max() < 1.5e-3
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(BIN, "test_2d_dic_fftcc_nr1")), reason="example binary not built")
+@pytest.mark.skipif(not os.path.exists(os.path.join(REF_BIN, "test_2d_dic_fftcc_nr1")), reason=REF_MISSING)
 def test_reference_2d_nr_example_runs_unchanged(tmp_path):
     """examples/test_2d_dic_fftcc_nr1.cpp of the reference (FFTCC2D -> NR2D1 -> Strain), compiled unchanged."""
     data = tmp_path / "d:" / "dic_tests" / "2d_dic"
     data.mkdir(parents=True)
     for name in ("oht_cfrp_0.bmp", "oht_cfrp_4.bmp"):
         shutil.copyfile(os.path.join(util.GOLDEN, name), data / name)
-    out = subprocess.run([os.path.join(BIN, "test_2d_dic_fftcc_nr1")], cwd=tmp_path, stdin=subprocess.DEVNULL,
+    out = subprocess.run([os.path.join(REF_BIN, "test_2d_dic_fftcc_nr1")], cwd=tmp_path, stdin=subprocess.DEVNULL,
                          capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stdout + out.stderr
     header, tab = _read_table(data / "oht_cfrp_4_fftcc_nr1_r16.csv")
@@ -125,7 +128,7 @@ def test_reference_2d_nr_example_runs_unchanged(tmp_path):
     assert np.percentile(np.abs(mb[conv][:, 10:13] - band[conv][:, 5:8]).max(1), 50) < 2e-5
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(BIN, "test_2d_dic_strain")), reason="example binary not built")
+@pytest.mark.skipif(not os.path.exists(os.path.join(REF_BIN, "test_2d_dic_strain")), reason=REF_MISSING)
 def test_reference_2d_strain_example_runs_unchanged(tmp_path):
     """examples/test_2d_dic_strain.cpp: loadTable2D -> Strain -> saveTable2D / saveMap2D, compiled unchanged.  Its input
     table is written here from the band fixture (the columns saveTable2D writes)."""
@@ -137,7 +140,7 @@ def test_reference_2d_strain_example_runs_unchanged(tmp_path):
         f.write("x,y,u,v,u0,v0,ZNCC,iteration,convergence,feature,exx,eyy,exy,subset_rx,subset_ry,\n")
         for p in q:
             f.write("%g,%g,%.8f,%.8f,0,0,%.8f,3,0.0001,0,0,0,0,16,16,\n" % (p[0], p[1], p[2], p[8], p[16]))
-    out = subprocess.run([os.path.join(BIN, "test_2d_dic_strain")], cwd=tmp_path, stdin=subprocess.DEVNULL,
+    out = subprocess.run([os.path.join(REF_BIN, "test_2d_dic_strain")], cwd=tmp_path, stdin=subprocess.DEVNULL,
                          capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stdout + out.stderr
     _, tab = _read_table(data / "oht_cfrp_4_fftcc_icgn1_r16.csv")
@@ -171,7 +174,7 @@ def _write_tiff_stack(path, vol):
         f.write(out)
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(BIN, "test_dvc_strain")), reason="example binary not built")
+@pytest.mark.skipif(not os.path.exists(os.path.join(REF_BIN, "test_dvc_strain")), reason=REF_MISSING)
 def test_reference_dvc_strain_example_runs_unchanged(tmp_path):
     """examples/test_dvc_strain.cpp: Image3D(.tif) for the dimensions, loadTable3D -> Strain -> saveTable3D."""
     data = tmp_path / "d:" / "dic_tests" / "dvc"
@@ -184,7 +187,7 @@ def test_reference_dvc_strain_example_runs_unchanged(tmp_path):
         for p in q:
             f.write("%g,%g,%g,%.8f,%.8f,%.8f,0,0,0,%.8f,5,0.0001,0," % (p[0], p[1], p[2], p[3], p[7], p[11], p[18])
                     + "0,0,0,0,0,0,0,0,0,0,0,0,0,0,0,16,16,16,\n")
-    out = subprocess.run([os.path.join(BIN, "test_dvc_strain")], cwd=tmp_path, stdin=subprocess.DEVNULL,
+    out = subprocess.run([os.path.join(REF_BIN, "test_dvc_strain")], cwd=tmp_path, stdin=subprocess.DEVNULL,
                          capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stdout + out.stderr
     _, tab = _read_table(data / "Torus_def_sift_icgn1_r16.csv")
@@ -194,7 +197,7 @@ def test_reference_dvc_strain_example_runs_unchanged(tmp_path):
     assert (data / "Torus_def_strain_r30_time.csv").exists()
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(BIN, "test_3d_dic_strain")), reason="example binary not built")
+@pytest.mark.skipif(not os.path.exists(os.path.join(REF_BIN, "test_3d_dic_strain")), reason=REF_MISSING)
 def test_reference_stereo_strain_example_runs_unchanged(tmp_path):
     """examples/test_3d_dic_strain.cpp: Image2D(.tif) for the size, loadTable2DS -> Strain(POI2DS) -> saveTable2DS."""
     data = tmp_path / "d:" / "dic_tests" / "3d_dic"
@@ -206,7 +209,7 @@ def test_reference_stereo_strain_example_runs_unchanged(tmp_path):
         f.write(cols + ",\n")
         for p in q:
             f.write(",".join("%.9g" % v for v in p[:20]) + ",0,0,0,0,0,0,16,16,\n")
-    out = subprocess.run([os.path.join(BIN, "test_3d_dic_strain")], cwd=tmp_path, stdin=subprocess.DEVNULL,
+    out = subprocess.run([os.path.join(REF_BIN, "test_3d_dic_strain")], cwd=tmp_path, stdin=subprocess.DEVNULL,
                          capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stdout + out.stderr
     header, tab = _read_table(data / "GT4-0273_0_epipolar_sift_r16.csv")
@@ -217,7 +220,7 @@ def test_reference_stereo_strain_example_runs_unchanged(tmp_path):
     assert np.median(d) < 2e-5 and d.max() < 1e-3
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(BIN, "test_dvc_fftcc_icgn1")), reason="example binary not built")
+@pytest.mark.skipif(not os.path.exists(os.path.join(REF_BIN, "test_dvc_fftcc_icgn1")), reason=REF_MISSING)
 def test_reference_dvc_example_runs_unchanged(tmp_path):
     """examples/test_dvc_fftcc_icgn1.cpp of the reference (north_star's second acceptance program: FFTCC3D -> ICGN3D1 with 61^3
     subvolumes on al_foam4_{0,1}.bin, 7 x 7 x 117 POIs), compiled unchanged against the shim.  The example hard-codes
@@ -235,7 +238,7 @@ def test_reference_dvc_example_runs_unchanged(tmp_path):
         with open(data / name, "wb") as f:
             np.array([100, 100, 706], np.int32).tofile(f)  # dim_x, dim_y, dim_z header, src/oc_image.cpp:76-110
             vol.tofile(f)
-    out = subprocess.run([os.path.join(BIN, "test_dvc_fftcc_icgn1")], cwd=tmp_path, stdin=subprocess.DEVNULL,
+    out = subprocess.run([os.path.join(REF_BIN, "test_dvc_fftcc_icgn1")], cwd=tmp_path, stdin=subprocess.DEVNULL,
                          capture_output=True, text=True, timeout=600)
     assert out.returncode == 0, out.stdout + out.stderr
     assert "5733 POIs" in out.stdout
@@ -254,24 +257,24 @@ def test_reference_dvc_example_runs_unchanged(tmp_path):
     assert (data / "al_foam4_1_fftcc_icgn1_r30_time.csv").exists()
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(BIN, "shim_bench")), reason="shim_bench not built")
+@pytest.mark.skipif(not os.path.exists(os.path.join(BIN, "dic_fftcc_icgn1_demo")), reason="demo binary not built")
 def test_shim_multi_device_matches_single_device(tmp_path):
     """The C++ shim with OPENCORR_B200_DEVICES=all (a GROUP context: FFTCC2D::compute / ICGN2D1::compute shard their
-    std::vector<POI2D> over every visible GPU inside the C ABI) returns the same records as on one GPU: the unchanged 2D example
-    writes byte-identical result tables either way.  (On a one-GPU box the group has one member.)"""
+    std::vector<POI2D> over every visible GPU inside the C ABI) returns the same records as on one GPU: the shim demo (the 2D
+    example's calls: FFTCC2D, ICGN2D1, IO2D::saveTable2D) writes byte-identical result tables either way.  (On a one-GPU box
+    the group has one member.)"""
     tables = []
     for env_extra in ({"OPENCORR_B200_DEVICE": "0"}, {"OPENCORR_B200_DEVICES": "all"}):
-        root = tmp_path / ("run_" + "_".join(env_extra.values()))
-        data = root / "d:" / "dic_tests" / "2d_dic"
-        data.mkdir(parents=True)
-        for name in ("oht_cfrp_0.bmp", "oht_cfrp_4.bmp"):
-            shutil.copyfile(os.path.join(util.GOLDEN, name), data / name)
+        out_csv = tmp_path / ("run_%s.csv" % "_".join(env_extra.values()))
         env = dict(os.environ)
         env.pop("OPENCORR_B200_DEVICE", None)
         env.pop("OPENCORR_B200_DEVICES", None)
         env.update(env_extra)
-        out = subprocess.run([os.path.join(BIN, "test_2d_dic_fftcc_icgn1")], cwd=root, stdin=subprocess.DEVNULL, capture_output=True, text=True,
-                             timeout=300, env=env)
+        out = subprocess.run([os.path.join(BIN, "dic_fftcc_icgn1_demo"), os.path.join(util.GOLDEN, "oht_cfrp_0.bmp"),
+                              os.path.join(util.GOLDEN, "oht_cfrp_4.bmp"), str(out_csv), "16", "2"],
+                             stdin=subprocess.DEVNULL, capture_output=True, text=True, timeout=300, env=env)
         assert out.returncode == 0, out.stdout + out.stderr
-        tables.append(open(data / "oht_cfrp_4_fftcc_icgn1_r16.csv", "rb").read())
+        tables.append(out_csv.read_bytes())
+    _, tab = _read_table(out_csv)
+    assert tab.shape[0] > 30000 and (tab[:, 6] > 0.9).mean() > 0.9
     assert tables[0] == tables[1]

@@ -95,21 +95,22 @@ def test_dvc_golden_tables():
         assert dz < tol_z, (exact, dz)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/examples/2d_dic"), reason="reference checkout not mounted")
 def test_2d_full_table_against_reference_checkout():
-    """All 30 000 POIs of the shipped table (only where the reference checkout is available)."""
-    tab = np.genfromtxt("/root/reference/examples/2d_dic/oht_cfrp_4_fftcc_icgn1_r16.csv", delimiter=",", skip_header=1)
+    """All 30 000 POIs of the shipped table (the columns the oracle is checked on, tests/golden/oht_cfrp_4_fftcc_icgn1_r16_full.npz)."""
+    g = np.load(os.path.join(util.GOLDEN, "oht_cfrp_4_fftcc_icgn1_r16_full.npz"))
+    xy, u0v0, it, uv, zncc = g["xy"], g["u0v0"], g["iteration"], g["uv"], g["zncc"]
+    assert len(xy) == 30000
     ref, tar = util.oht_cfrp_pair()
-    q = make_poi2d(tab[:, 0:2])
+    q = make_poi2d(xy.astype(np.float32))
     o = Oracle2D(ref, tar)
     o.fftcc2d(q, 16, 16)
     o.icgn2d1(q, 16, 16, 0.001, 10)
-    guess_same = (q[:, 14] == tab[:, 4]) & (q[:, 15] == tab[:, 5])
+    guess_same = (q[:, 14] == u0v0[:, 0]) & (q[:, 15] == u0v0[:, 1])
     assert list(np.where(~guess_same)[0]) == [22154, 22472, 22557]  # exact ties of the correlation map, see test_2d_fftcc_ties
-    ok = guess_same & (tab[:, 7] < 10) & (q[:, 17] == tab[:, 7])
+    ok = guess_same & (it < 10) & (q[:, 17] == it)
     assert ok.sum() >= 28000
-    assert np.abs(q[ok][:, [2, 8]] - tab[ok][:, [2, 3]]).max() < 5e-5
-    assert np.abs(q[ok, 16] - tab[ok, 6]).max() < 2e-6
+    assert np.abs(q[ok][:, [2, 8]] - uv[ok]).max() < 5e-5
+    assert np.abs(q[ok, 16] - zncc[ok]).max() < 2e-6
 
 
 def test_2d_iclm_golden_table():
