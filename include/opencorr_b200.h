@@ -101,6 +101,16 @@ int ocb_use_own_stream(ocb_ctx* ctx);
 int ocb_sync(ocb_ctx* ctx);
 /* Number of kernels this context has launched since creation (bench.py "gpu_launches"). */
 long long ocb_launch_count(const ocb_ctx* ctx);
+/* Which kernel the most recent FFT-CC 2D/3D, IC-GN/IC-LM 2D or ICGN3D1 call of this context launched, as space-separated
+ * key=value pairs, so that a caller can tell which specialisation served its queue:
+ *   "op=icgn2d np=6 rc=0 lm=0 wpp=1 tm=1 tma=1 grid=... threads=128"   (rc: compile-time subset radius, 0 = generic;
+ *                                                                      wpp: warps per POI; tm: Tensor-Memory variant)
+ *   "op=icgn3d rc=0 threads=256 slab_k=... nslab=... tma=1 grid=..."    (slab_k: layers per z-slab, nslab: slabs)
+ *   "op=fftcc2d kernel=w32|reg|generic n=32 tma=1"                     (n: window points along x)
+ * A host-queue 2D call of 16384 POIs or more goes out in four pipelined chunks, each its own launch: the description is
+ * then that of the last chunk.  Never NULL; empty before the first such launch, and on a group context (ocb_member()
+ * gives the member contexts, which keep their own). */
+const char* ocb_last_launch(const ocb_ctx* ctx);
 
 /* ---- images: DIC::setImages / DVC::setImages (src/oc_dic.cpp:22-26,44-48) ----------------- */
 /* Host buffers; copied to the device (H2D on the context's stream). */

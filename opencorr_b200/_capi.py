@@ -38,6 +38,7 @@ SIGNATURES = {
     "ocb_use_own_stream": (_i, [_vp]),
     "ocb_sync": (_i, [_vp]),
     "ocb_launch_count": (ctypes.c_longlong, [_vp]),
+    "ocb_last_launch": (ctypes.c_char_p, [_vp]),
     "ocb_set_images_2d": (_i, [_vp, _vp, _vp, _i, _i, _i]),
     "ocb_set_images_3d": (_i, [_vp, _vp, _vp, _i, _i, _i]),
     "ocb_set_images_2d_u8": (_i, [_vp, _vp, _vp, _i, _i]),

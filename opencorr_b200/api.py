@@ -151,6 +151,16 @@ class Engine:
     def launch_count(self):
         return int(self._lib.ocb_launch_count(self._ctx))
 
+    def last_launch(self):
+        """The kernel the most recent FFT-CC / IC-GN / IC-LM / ICGN3D1 call launched (include/opencorr_b200.h
+        ocb_last_launch), e.g. {"op": "icgn2d", "rc": 0, "tm": 1, ...}; numbers come back as int.  {} before any launch."""
+        text = self._lib.ocb_last_launch(self._ctx).decode("utf-8", "replace")
+        out = {}
+        for item in text.split():
+            key, _, value = item.partition("=")
+            out[key] = int(value) if value.lstrip("-").isdigit() else value
+        return out
+
     # hot path, host POI queues -------------------------------------------------------------------
     def fftcc2d(self, q, rx, ry):
         _check_queue(q, POI2D_FLOATS)

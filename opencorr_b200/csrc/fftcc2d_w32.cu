@@ -199,7 +199,7 @@ __global__ void __launch_bounds__(FFTW32_WARPS * 32) fftcc2d_w32_kernel(Image2D 
 	}
 }
 
-int fftcc2d_w32_launch(const Image2D& img, float* d_pois, size_t n, int sm_count, cudaStream_t stream, cudaError_t* err) {
+int fftcc2d_w32_launch(const Image2D& img, float* d_pois, size_t n, int sm_count, cudaStream_t stream, cudaError_t* err, int* use_tma_out) {
 	long long blocks_needed = ((long long)n + FFTW32_WARPS - 1) / FFTW32_WARPS;
 	long long grid = (long long)sm_count * 16;
 	if (grid > blocks_needed) grid = blocks_needed;
@@ -209,6 +209,7 @@ int fftcc2d_w32_launch(const Image2D& img, float* d_pois, size_t n, int sm_count
 	memset(&tm_tar, 0, sizeof(tm_tar));
 	const int dims[2] = { img.w, img.h }, box[2] = { FFTW32_BOX_W, 32 };
 	const int use_tma = !getenv("OCB_NO_TMA") && tma_make_map(&tm_ref, img.ref, 2, dims, box) && tma_make_map(&tm_tar, img.tar, 2, dims, box);
+	if (use_tma_out) *use_tma_out = use_tma;
 	fftcc2d_w32_kernel<<<(int)grid, FFTW32_WARPS * 32, 0, stream>>>(img, d_pois, (int)n, tm_ref, tm_tar, use_tma);
 	*err = cudaGetLastError();
 	return *err == cudaSuccess ? 0 : -2;

@@ -273,7 +273,8 @@ __global__ void __launch_bounds__(F3_WARPS * 32, 2) fftcc3d_w32_kernel(Image3D i
 
 int fftcc3d_w32_grid(int sm_count) { return sm_count * 2; }
 
-int fftcc3d_w32_launch(const Image3D& img, float* d_pois, size_t n, float2* scratch, int grid, cudaStream_t stream, cudaError_t* err) {
+int fftcc3d_w32_launch(const Image3D& img, float* d_pois, size_t n, float2* scratch, int grid, cudaStream_t stream, cudaError_t* err,
+	int* use_tma_out) {
 	if ((long long)grid > (long long)n) grid = (int)n;
 	if (grid < 1) grid = 1;
 	const size_t smem = (size_t)2 * F3_WARPS * F3_TILE * sizeof(float);
@@ -284,6 +285,7 @@ int fftcc3d_w32_launch(const Image3D& img, float* d_pois, size_t n, float2* scra
 	const int use_tma = !getenv("OCB_NO_TMA") && tma_make_map(&tm_ref, img.ref, 3, dims, box) && tma_make_map(&tm_tar, img.tar, 3, dims, box);
 	*err = cudaFuncSetAttribute(fftcc3d_w32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
 	if (*err != cudaSuccess) return -2;
+	if (use_tma_out) *use_tma_out = use_tma;
 	fftcc3d_w32_kernel<<<grid, F3_WARPS * 32, smem, stream>>>(img, d_pois, (int)n, scratch, tm_ref, tm_tar, use_tma);
 	*err = cudaGetLastError();
 	return *err == cudaSuccess ? 0 : -2;

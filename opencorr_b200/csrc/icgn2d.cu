@@ -1249,17 +1249,24 @@ __global__ void __launch_bounds__(TM ? 32 * ICGN2D_TM_WARPS : 32 * WPP, TM ? (NP
 // the self-resetting head and departure count of the one-warp-per-POI kernels).
 typedef void (*Icgn2dKernel)(Image2D, float*, int, int, int, float, float, int*, const CUtensorMap, const CUtensorMap, int, const float*, float, float, float);
 
+// *rc: the compile-time subset radius of the instantiation picked (0: any radius)
 template <int WPP>
-static Icgn2dKernel icgn2d_pick(int np, int rx, int ry, bool lm) {
+static Icgn2dKernel icgn2d_pick(int np, int rx, int ry, bool lm, int* rc) {
+	*rc = 0;
 	if (lm) return (np == 6) ? icgn2d_kernel<6, 0, true, WPP> : icgn2d_kernel<12, 0, true, WPP>;
-	if (np == 6) return (rx == 16 && ry == 16) ? icgn2d_kernel<6, 16, false, WPP> : icgn2d_kernel<6, 0, false, WPP>;
-	return (rx == 20 && ry == 20) ? icgn2d_kernel<12, 20, false, WPP> : icgn2d_kernel<12, 0, false, WPP>;
+	if (np == 6) {
+		if (rx == 16 && ry == 16) { *rc = 16; return icgn2d_kernel<6, 16, false, WPP>; }
+		return icgn2d_kernel<6, 0, false, WPP>;
+	}
+	if (rx == 20 && ry == 20) { *rc = 20; return icgn2d_kernel<12, 20, false, WPP>; }
+	return icgn2d_kernel<12, 0, false, WPP>;
 }
 
 size_t icgn2d_slab_bytes(int rx, int ry) { return (size_t)icgn2d_slab_floats(rx, ry, false, 1) * sizeof(float); }
 
 int icgn2d_launch(int np, const Image2D& img, float* d_pois, size_t n, int rx, int ry, float conv, float stop, int sm_count,
-	size_t smem_optin, int* d_counter, const float* d_center_offsets, const float* lm_damping, cudaStream_t stream, cudaError_t* err) {
+	size_t smem_optin, int* d_counter, const float* d_center_offsets, const float* lm_damping, cudaStream_t stream, cudaError_t* err,
+	LaunchInfo* info) {
 	const bool lm = lm_damping != nullptr;
 	// Warps per POI.  Measured on B200 (tools/ab_icgn2d.sh): with the GPU full, one warp per POI wins (config B 0.853 vs
 	// 0.906 ms, C 2.22 vs 2.43 ms, E 8.38 vs 8.87 ms) -- the second warp doubles the resident warps but also the per-POI
@@ -1298,11 +1305,13 @@ int icgn2d_launch(int np, const Image2D& img, float* d_pois, size_t n, int rx, i
 	const int dims[2] = { img.w, img.h };
 	const int box_ref[2] = { icgn2d_ref_w(rx), icgn2d_ref_h(ry) }, box_tar[2] = { icgn2d_tar_w(rx), icgn2d_tar_h(ry) };
 	const int use_tma = !getenv("OCB_NO_TMA") && tma_make_map(&tm_ref, img.ref, 2, dims, box_ref) && tma_make_map(&tm_tar, img.tar, 2, dims, box_tar);
-	Icgn2dKernel kern = wpp == 2 ? icgn2d_pick<2>(np, rx, ry, lm) : icgn2d_pick<1>(np, rx, ry, lm);
+	int rc = 0;
+	Icgn2dKernel kern = wpp == 2 ? icgn2d_pick<2>(np, rx, ry, lm, &rc) : icgn2d_pick<1>(np, rx, ry, lm, &rc);
 	int threads = wpp * 32;
 	if (use_tm) {
 		// (6-parameter kernels only: the 12-parameter ones need ~250 registers, which already limits them to 8 warps per SM)
-		kern = (rx == 16 && ry == 16) ? icgn2d_kernel<6, 16, false, 1, true> : icgn2d_kernel<6, 0, false, 1, true>;
+		rc = (rx == 16 && ry == 16) ? 16 : 0;
+		kern = rc == 16 ? icgn2d_kernel<6, 16, false, 1, true> : icgn2d_kernel<6, 0, false, 1, true>;
 		smem = tm_cta_smem;
 		threads = ICGN2D_TM_WARPS * 32;
 		blocks_per_sm = 512 / ICGN2D_TM_COLS; // Tensor Memory: 512 columns per SM
@@ -1319,6 +1328,11 @@ int icgn2d_launch(int np, const Image2D& img, float* d_pois, size_t n, int rx, i
 	if (use_tm && (long long)n < resident * ICGN2D_TM_WARPS) resident = ((long long)n + ICGN2D_TM_WARPS - 1) / ICGN2D_TM_WARPS;
 	int grid = (int)((long long)n < resident ? (long long)n : resident); // persistent: one wave, one POI per CTA (TM: per warp) at a time
 	if (grid < 1) grid = 1;
+	if (info) {
+		info->op = "icgn2d";
+		info->np = np; info->rc = rc; info->lm = lm; info->wpp = wpp; info->tm = use_tm; info->tma = use_tma;
+		info->grid = grid; info->threads = threads;
+	}
 	kern<<<grid, threads, smem, stream>>>(img, d_pois, (int)n, rx, ry, conv, stop, d_counter, tm_ref, tm_tar, use_tma, d_center_offsets,
 		lm ? lm_damping[0] : 0.f, lm ? lm_damping[1] : 0.f, lm ? lm_damping[2] : 0.f);
 	*err = cudaGetLastError();

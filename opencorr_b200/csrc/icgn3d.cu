@@ -739,7 +739,7 @@ __global__ void __launch_bounds__(THREADS, 512 / THREADS) icgn3d1_kernel(Image3D
 
 // Returns 0, -1 when even a one-layer slab does not fit in shared memory, -2 on a CUDA error.
 int icgn3d1_launch(const Image3D& img, float* d_pois, size_t n, int rx, int ry, int rz, float conv, float stop, int sm_count, size_t smem_optin,
-	int* d_counter, cudaStream_t stream, cudaError_t* err) {
+	int* d_counter, cudaStream_t stream, cudaError_t* err, LaunchInfo* info) {
 	const int sz = 2 * rz + 1;
 	const size_t layer = (size_t)icgn3d_tile_x(rx) * icgn3d_tile_y(ry) * sizeof(float);
 	const size_t fixed = 128 + sizeof(Icgn3dShared) + 1024; // barrier pad + static smem + per-CTA reservation
@@ -764,8 +764,14 @@ int icgn3d1_launch(const Image3D& img, float* d_pois, size_t n, int rx, int ry, 
 	const int use_tma = !getenv("OCB_NO_TMA") && tma_make_map(&tm, img.coef, 3, dims, box);
 	void (*kern)(Image3D, float*, int, int, int, int, float, float, int, int*, const CUtensorMap, int);
 	const int threads = ctas == 1 ? 512 : 256;
-	if (ctas == 1) kern = (rx == 30 && ry == 30 && rz == 30) ? icgn3d1_kernel<30, 512> : icgn3d1_kernel<0, 512>; // 61^3: the reference's own DVC example
-	else kern = (rx == 16 && ry == 16 && rz == 16) ? icgn3d1_kernel<16, 256> : icgn3d1_kernel<0, 256>;
+	int rc = 0;
+	if (ctas == 1) { // 61^3: the reference's own DVC example
+		if (rx == 30 && ry == 30 && rz == 30) rc = 30;
+		kern = rc == 30 ? icgn3d1_kernel<30, 512> : icgn3d1_kernel<0, 512>;
+	} else {
+		if (rx == 16 && ry == 16 && rz == 16) rc = 16;
+		kern = rc == 16 ? icgn3d1_kernel<16, 256> : icgn3d1_kernel<0, 256>;
+	}
 	*err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
 	if (*err != cudaSuccess) return -2;
 	*err = cudaMemsetAsync(d_counter, 0, sizeof(int), stream);
@@ -773,6 +779,10 @@ int icgn3d1_launch(const Image3D& img, float* d_pois, size_t n, int rx, int ry, 
 	long long grid = (long long)sm_count * ctas;
 	if (grid > (long long)n) grid = (long long)n;
 	if (grid < 1) grid = 1;
+	if (info) {
+		info->op = "icgn3d";
+		info->rc = rc; info->threads = threads; info->slab_k = slab_k; info->nslab = nslab; info->tma = use_tma; info->grid = (int)grid;
+	}
 	kern<<<(int)grid, threads, smem, stream>>>(img, d_pois, (int)n, rx, ry, rz, conv, stop, slab_k, d_counter, tm, use_tma);
 	*err = cudaGetLastError();
 	return *err == cudaSuccess ? 0 : -2;

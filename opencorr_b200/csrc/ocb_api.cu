@@ -119,6 +119,7 @@ struct ocb_ctx {
 	cudaStream_t stream = nullptr;
 	std::string last_error;
 	long long launches = 0;
+	std::string last_launch; // ocb_last_launch
 
 	// 2D images
 	float* own_ref2 = nullptr;
@@ -177,6 +178,30 @@ static int set_error(ocb_ctx* ctx, int code, const char* fmt, ...) {
 	g_last_error = buf;
 	if (ctx) ctx->last_error = buf;
 	return code;
+}
+
+// Keep a key=value description of the kernel launch that just went out (ocb_last_launch).
+static void record_launch(ocb_ctx* ctx, const ocb::LaunchInfo& li) {
+	char buf[192];
+	const std::string op = li.op;
+	if (op == "icgn2d")
+		snprintf(buf, sizeof(buf), "op=icgn2d np=%d rc=%d lm=%d wpp=%d tm=%d tma=%d grid=%d threads=%d", li.np, li.rc, li.lm, li.wpp, li.tm,
+			li.tma, li.grid, li.threads);
+	else if (op == "icgn3d")
+		snprintf(buf, sizeof(buf), "op=icgn3d rc=%d threads=%d slab_k=%d nslab=%d tma=%d grid=%d", li.rc, li.threads, li.slab_k, li.nslab,
+			li.tma, li.grid);
+	else
+		snprintf(buf, sizeof(buf), "op=%s kernel=%s n=%d tma=%d", li.op, li.kernel, li.n, li.tma);
+	ctx->last_launch = buf;
+}
+
+static ocb::LaunchInfo fftcc_info(const char* op, const char* kernel, int n, int tma) {
+	ocb::LaunchInfo li;
+	li.op = op;
+	li.kernel = kernel;
+	li.n = n;
+	li.tma = tma;
+	return li;
 }
 
 #define OCB_CUDA(ctx, call)                                                                                   \
@@ -674,6 +699,8 @@ void ocb_destroy(ocb_ctx* ctx) {
 
 const char* ocb_last_error(const ocb_ctx* ctx) { return ctx ? ctx->last_error.c_str() : g_last_error.c_str(); }
 
+const char* ocb_last_launch(const ocb_ctx* ctx) { return ctx ? ctx->last_launch.c_str() : ""; }
+
 int ocb_set_stream(ocb_ctx* ctx, void* cuda_stream) {
 	if (!ctx) return set_error(nullptr, OCB_ERR_ARG, "null context");
 	OCB_NO_GROUP(ctx, "set_stream");
@@ -876,9 +903,11 @@ int ocb_fftcc2d_dev(ocb_ctx* ctx, void* d_poi2d, size_t n, int rx, int ry) {
 	if (ensure_device(ctx)) return OCB_ERR_CUDA;
 	if (rx == 16 && ry == 16 && !getenv("OCB_FFTCC2D_GENERIC")) { // specialised register-FFT kernel for the 32x32 window
 		cudaError_t err32;
-		if (ocb::fftcc2d_w32_launch(ctx->img2, (float*)d_poi2d, n, ctx->sm_count, ctx->stream, &err32))
+		int tma = 0;
+		if (ocb::fftcc2d_w32_launch(ctx->img2, (float*)d_poi2d, n, ctx->sm_count, ctx->stream, &err32, &tma))
 			return set_error(ctx, OCB_ERR_CUDA, "fftcc2d launch failed: %s", cudaGetErrorString(err32));
 		ctx->launches++;
+		record_launch(ctx, fftcc_info("fftcc2d", "w32", 32, tma));
 		return OCB_OK;
 	}
 	if (rx == ry && ocb::fftcc2d_reg_supported(rx) && !getenv("OCB_FFTCC2D_GENERIC")) { // thread-per-row register FFTs, N = 2^a 3^b 5^c <= 64
@@ -886,6 +915,7 @@ int ocb_fftcc2d_dev(ocb_ctx* ctx, void* d_poi2d, size_t n, int rx, int ry) {
 		if (ocb::fftcc2d_reg_launch(ctx->img2, (float*)d_poi2d, n, rx, ctx->sm_count, ctx->stream, &errr))
 			return set_error(ctx, OCB_ERR_CUDA, "fftcc2d launch failed: %s", cudaGetErrorString(errr));
 		ctx->launches++;
+		record_launch(ctx, fftcc_info("fftcc2d", "reg", 2 * rx, 0));
 		return OCB_OK;
 	}
 	ocb::FftAxis ax, ay;
@@ -901,6 +931,7 @@ int ocb_fftcc2d_dev(ocb_ctx* ctx, void* d_poi2d, size_t n, int rx, int ry) {
 	if (ocb::fftcc2d_launch(ctx->img2, (float*)d_poi2d, n, rx, ry, ax, ay, twx, twy, ctx->sm_count, ctx->stream, &err))
 		return set_error(ctx, OCB_ERR_CUDA, "fftcc2d launch failed: %s", cudaGetErrorString(err));
 	ctx->launches++;
+	record_launch(ctx, fftcc_info("fftcc2d", "generic", 2 * rx, 0));
 	return OCB_OK;
 }
 
@@ -934,9 +965,11 @@ int ocb_fftcc3d_dev(ocb_ctx* ctx, void* d_poi3d, size_t n, int rx, int ry, int r
 			ctx->fft_scratch_elems = need32;
 		}
 		cudaError_t err32;
-		if (ocb::fftcc3d_w32_launch(ctx->img3, (float*)d_poi3d, n, ctx->fft_scratch, grid32, ctx->stream, &err32))
+		int tma = 0;
+		if (ocb::fftcc3d_w32_launch(ctx->img3, (float*)d_poi3d, n, ctx->fft_scratch, grid32, ctx->stream, &err32, &tma))
 			return set_error(ctx, OCB_ERR_CUDA, "fftcc3d launch failed: %s", cudaGetErrorString(err32));
 		ctx->launches++;
+		record_launch(ctx, fftcc_info("fftcc3d", "w32", 32, tma));
 		return OCB_OK;
 	}
 	if (rx == ry && ry == rz && ocb::fftcc3d_reg_supported(rx) && !getenv("OCB_FFTCC3D_GENERIC")) { // register FFT codelets, N = 2^a 3^b 5^c <= 64
@@ -955,6 +988,7 @@ int ocb_fftcc3d_dev(ocb_ctx* ctx, void* d_poi3d, size_t n, int rx, int ry, int r
 		if (ocb::fftcc3d_reg_launch(ctx->img3, (float*)d_poi3d, n, rx, ctx->fft_scratch, gridr, ctx->stream, &errr))
 			return set_error(ctx, OCB_ERR_CUDA, "fftcc3d launch failed: %s", cudaGetErrorString(errr));
 		ctx->launches++;
+		record_launch(ctx, fftcc_info("fftcc3d", "reg", 2 * rx, 0));
 		return OCB_OK;
 	}
 	ocb::FftAxis ax, ay, az;
@@ -981,6 +1015,7 @@ int ocb_fftcc3d_dev(ocb_ctx* ctx, void* d_poi3d, size_t n, int rx, int ry, int r
 	if (ocb::fftcc3d_launch(ctx->img3, (float*)d_poi3d, n, rx, ry, rz, ax, ay, az, twx, twy, twz, ctx->fft_scratch, grid, ctx->stream, &err))
 		return set_error(ctx, OCB_ERR_CUDA, "fftcc3d launch failed: %s", cudaGetErrorString(err));
 	ctx->launches++;
+	record_launch(ctx, fftcc_info("fftcc3d", "generic", 2 * rx, 0));
 	return OCB_OK;
 }
 
@@ -1021,11 +1056,13 @@ static int icgn2d_dev(ocb_ctx* ctx, int np, void* d_poi2d, size_t n, int rx, int
 	if (n > 0x7fffffffull) return set_error(ctx, OCB_ERR_ARG, "icgn2d: too many POIs in one call");
 	if (ensure_device(ctx)) return OCB_ERR_CUDA;
 	cudaError_t err = cudaSuccess;
+	ocb::LaunchInfo li;
 	int rc = ocb::icgn2d_launch(np, ctx->img2, (float*)d_poi2d, n, rx, ry, conv, stop, ctx->sm_count, ctx->smem_optin, ctx->d_counter, d_offsets, lm_damping,
-		ctx->stream, &err);
+		ctx->stream, &err, &li);
 	if (rc == -1) return set_error(ctx, OCB_ERR_UNSUPPORTED, "icgn2d: subset radius (%d,%d) exceeds the shared-memory design limit", rx, ry);
 	if (rc) return set_error(ctx, OCB_ERR_CUDA, "icgn2d launch failed: %s", cudaGetErrorString(err));
 	ctx->launches++;
+	record_launch(ctx, li);
 	return OCB_OK;
 }
 
@@ -1335,11 +1372,13 @@ int ocb_icgn3d1_dev(ocb_ctx* ctx, void* d_poi3d, size_t n, int rx, int ry, int r
 	if ((size_t)(2 * rx + 1) * (2 * ry + 1) * (2 * rz + 1) > 0x3fffffffull) return set_error(ctx, OCB_ERR_UNSUPPORTED, "icgn3d1: subset too large");
 	if (ensure_device(ctx)) return OCB_ERR_CUDA;
 	cudaError_t err = cudaSuccess;
+	ocb::LaunchInfo li;
 	const int rc3 = ocb::icgn3d1_launch(ctx->img3, (float*)d_poi3d, n, rx, ry, rz, conv, stop, ctx->sm_count, ctx->smem_optin, ctx->d_counter + 1,
-		ctx->stream, &err);
+		ctx->stream, &err, &li);
 	if (rc3 == -1) return set_error(ctx, OCB_ERR_UNSUPPORTED, "icgn3d1: subset radius (%d,%d,%d) exceeds the shared-memory design limit", rx, ry, rz);
 	if (rc3) return set_error(ctx, OCB_ERR_CUDA, "icgn3d1 launch failed: %s", cudaGetErrorString(err));
 	ctx->launches++;
+	record_launch(ctx, li);
 	return OCB_OK;
 }
 

@@ -184,6 +184,8 @@ def test_icgn2d2_matches_oracle(engine, r):
     icgn.set_images(ref, tar)
     icgn.prepare()
     icgn.compute(q_gpu)
+    got = engine.last_launch()  # 192 POIs cannot fill the GPU: two warps per POI; r = 20 has its own instantiation
+    assert got.get("np") == 12 and got.get("wpp") == 2 and got.get("rc") == (20 if r == 20 else 0), "r=%d: ran %s" % (r, got)
     o.icgn2d2(q_cpu, r, r, 0.001, 10)
     stats = util.compare_2d(q_gpu, q_cpu, "icgn2d2 r=%d" % r, max_iter_mismatch_frac=0.03)
     assert stats["n_compared"] >= 0.9 * len(q)
@@ -286,6 +288,8 @@ def test_icgn2d1_image_width_not_multiple_of_four(engine, width):
     icgn.set_images(ref, tar)
     icgn.prepare()
     icgn.compute(q_gpu)
+    got = engine.last_launch()
+    assert got.get("rc") == 16 and got.get("tma") == 0 and got.get("wpp") == 2, "width %d: ran %s" % (width, got)
     o.icgn2d1(q_cpu, 16, 16, 0.001, 10)
     stats = util.compare_2d(q_gpu, q_cpu, "width %d" % width, max_iter_mismatch_frac=0.03)
     assert stats["n_compared"] >= 0.9 * len(q)
@@ -462,7 +466,8 @@ def test_iclm2d1_golden_table(engine):
 @pytest.mark.parametrize("order", [1, 2])
 def test_icgn2d_warps_per_poi_variants(engine, cfg_a, monkeypatch, wpp, order):
     """The launch picks one or two warps per POI from the queue length (icgn2d.cu icgn2d_launch); both code paths must
-    meet the same parity bar, also with sentinels, an odd row split and the LM variant."""
+    meet the same parity bar, also with sentinels, an odd row split and the LM variant of the same order (ICLM2D1,
+    ICLM2D2: icgn2d_kernel<6 or 12, 0, true, WPP>)."""
     monkeypatch.setenv("OCB_ICGN2D_WPP", wpp)
     ref, tar, xy, _ = cfg_a
     o = Oracle2D(ref, tar)
@@ -476,16 +481,22 @@ def test_icgn2d_warps_per_poi_variants(engine, cfg_a, monkeypatch, wpp, order):
         ic.prepare()
         ic.compute(a)
         (o.icgn2d1 if order == 1 else o.icgn2d2)(b, rx, ry, 0.001, 10)
+        got = engine.last_launch()
+        assert got.get("np") == 6 * order and got.get("wpp") == int(wpp) and got.get("lm") == 0 and got.get("tm") == 0, \
+            "wpp=%s order=%d: ran %s" % (wpp, order, got)
         util.compare_2d(a, b, "wpp=%s order=%d r=(%d,%d)" % (wpp, order, rx, ry), order=order)
         assert a[-1, 16] == -3 and a[-2, 16] == -3
-    lm = ob.ICLM2D1(16, 16, 0.001, 10, engine=engine)
+    lm = (ob.ICLM2D1 if order == 1 else ob.ICLM2D2)(16, 16, 0.001, 10, engine=engine)
     lm.set_images(ref, tar)
     lm.prepare()
     q = ob.make_poi2d(xy)
     o.fftcc2d(q, 16, 16)
     a, b = q.copy(), q.copy()
     lm.compute(a)
-    o.iclm2d(1, b, 16, 16, 0.001, 10)
+    got = engine.last_launch()
+    assert got.get("np") == 6 * order and got.get("wpp") == int(wpp) and got.get("lm") == 1 and got.get("rc") == 0, \
+        "ICLM wpp=%s order=%d: ran %s" % (wpp, order, got)
+    o.iclm2d(order, b, 16, 16, 0.001, 10)
     same = a[:, 17] == b[:, 17]
     assert same.mean() > 0.97
     assert np.abs(a[same][:, [2, 8]] - b[same][:, [2, 8]]).max() < 1e-4

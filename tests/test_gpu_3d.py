@@ -52,11 +52,13 @@ def test_fftcc3d_matches_oracle(engine, vol, r):
     assert (q_cpu[:, 18] > 0.3).all()
 
 
-@pytest.mark.parametrize("r", [4, 5, 6, 9, 10, 12, 18, 20])
+@pytest.mark.parametrize("r", [4, 5, 6, 9, 10, 12, 18, 20, 24, 25, 27, 32])
 def test_fftcc3d_register_kernels(engine, r):
-    """The cubic windows served by fftcc3d_reg.cu (one thread per 1D transform, register codelets); r = 8, 15 and 30 are
-    covered by the tests above / the golden DVC table.  Includes a POI too close to the border (left untouched) and a
-    non-zero incoming guess."""
+    """Every cubic window fftcc3d_reg.cu serves through the dispatch (one thread per 1D transform, register codelets,
+    OCB_F3R_SIZES) apart from r = 15 and 30, which test_fftcc3d_matches_oracle and the golden DVC table cover: N = 2r
+    from 8 to 64, with 2 * 5^2 and 2 * 3^3 among them.  r = 16 takes fftcc3d_w32 instead (test_fftcc3d_w32_specialised_kernel),
+    so fftcc3d_reg_kernel<32> is never launched.  Includes a POI too close to the border (left untouched) and a non-zero
+    incoming guess."""
     ref, tar = synth.speckle_pair_3d(96, 88, 80)
     c = np.array([[48, 44, 40], [50, 41, 38], [44, 46, 42], [3, 44, 40]], np.float32)
     if r > 12:
@@ -68,8 +70,12 @@ def test_fftcc3d_register_kernels(engine, r):
     f = ob.FFTCC3D(r, r, r, engine=engine)
     f.set_images(ref, tar)
     f.compute(q_gpu)
+    got = engine.last_launch()
+    assert got.get("op") == "fftcc3d" and got.get("kernel") == "reg" and got.get("n") == 2 * r, \
+        "r=%d: expected kernel=reg n=%d, ran %s" % (r, 2 * r, got)
     o = Oracle3D(ref, tar)
     o.fftcc3d(q_cpu, r, r, r, exact=True)
+    assert q_cpu[0, 18] > 0.3  # the window (and the guess) fit the volume: a real correlation, not a skipped POI
     assert np.array_equal(q_gpu[:, [3, 7, 11, 15, 16, 17]], q_cpu[:, [3, 7, 11, 15, 16, 17]])
     assert np.abs(q_gpu[:, 18] - q_cpu[:, 18]).max() < 1e-5
     assert q_gpu[-1, 18] == 0 and np.all(q_gpu[-1, 3:15] == 0)

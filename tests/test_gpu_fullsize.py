@@ -40,6 +40,10 @@ def test_full_size_2d(engine, name):
         return q
 
     q = run(xy)
+    # the specialisation each config exists to measure (the record is that of the last of the four pipelined chunks)
+    want = dict(np=12, rc=20, wpp=1, tm=0) if order == 2 else dict(np=6, rc=16, wpp=1, tm=1)
+    got = engine.last_launch()
+    assert all(got.get(k) == v for k, v in want.items()), "config %s: expected %s, ran %s" % (name, want, got)
     # (1) every POI converged onto the analytic displacement field (loose: the field is not exactly affine per subset)
     assert (q[:, 16] > 0.9).all()
     u_true, v_true = synth.displacement_2d(xy[:, 0], xy[:, 1], cfg["size"][0], cfg["size"][1], second_order=(order == 2))
